@@ -4,6 +4,7 @@
   python bench.py --gpus N --steps K --warmup W            # our arm (fused sm_100a Linear4bit), 1 process / GPU
   python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle dequant + CPU matmul)
   python bench.py --impl unfused ...                       # bnb-equivalent GPU restatement (dequant kernel + cuBLAS)
+  python bench.py ... --dump-outputs DIR                   # also save the last timed step's outputs as DIR/*.npy
 
 A "step" = one optimizer step on ONE synthetic OASST-shaped sample per GPU: forward (32 checkpointed decoder
 layers, 7 Linear4bit+LoRA each), backward (checkpoint recompute + dX), DDP allreduce of LoRA grads (N>1),
@@ -55,7 +56,14 @@ def parse_args():
                          "Measured slower than one allreduce after backward at 2 GPUs (96.7 vs 95.3 ms): the NCCL kernels take SMs from "
                          "the persistent NF4 kernel, whose static schedule then needs a second round — see DESIGN.md 5")
     ap.add_argument("--cpu-reps", type=int, default=3, help="repetitions of the CPU sample (median reported)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32): the loss, and a "
+                         "fixed seeded sample of the adapter weights after the update and of their clipped gradients")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        # that arm times one decoder layer's Linear4bit path on the host with random packed weights: it runs no training step
+        ap.error("--dump-outputs needs a GPU arm (--impl ours, unfused or bf16): --impl reference runs no training step")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------
@@ -248,6 +256,30 @@ def run_reference_arm(args):
 # ---------------------------------------------------------------------------------------------
 # GPU arms
 # ---------------------------------------------------------------------------------------------
+DUMP_SAMPLE = 1 << 22   # sampled elements per dumped array: 16 MB as float32, so the files stay well under 64 MB in all
+
+
+def dump_outputs(out_dir: str, loss, params, grads) -> None:
+    """What a training step hands back to its caller: the loss, the adapter weights after the optimizer update and the
+    gradients the update applied, clipped to norm 0.3 (`grads`: laid out like `params`).  With --grad-accum the loss is the
+    last micro-batch's, divided by the micro-batch count as it was backpropagated.  Llama-2-7B has 160 M adapter values, so
+    larger outputs are sampled at positions drawn from a fixed seed: the same positions in every run, for element-wise
+    comparison."""
+    import numpy as np
+    import torch
+
+    weights = torch.cat([p.detach().reshape(-1) for p in params])
+    n = weights.numel()
+    if n <= DUMP_SAMPLE:
+        idx = torch.arange(n, device=weights.device)
+    else:
+        idx = torch.randint(0, n, (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).unique().to(weights.device)
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"loss": loss.detach().reshape(1), "lora_weights": weights[idx], "lora_grads": grads.detach().reshape(-1)[idx]}
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.float().cpu().numpy())
+
+
 def run_gpu_arm(args):
     import torch
     import torch.distributed as dist
@@ -277,6 +309,9 @@ def run_gpu_arm(args):
     shape = SHAPES[args.model]
     accum = max(1, args.grad_accum)
     torch.backends.cuda.matmul.allow_tf32 = True  # qlora.py:70
+    # lora_A, embed_tokens and lm_head are initialised from the global RNG: seed it so that every run, and every rank, starts
+    # from the same weights
+    torch.manual_seed(1234)
     model = LlamaQLoRA(shape, device, lora_r=args.lora_r, lora_alpha=16, lora_dropout=args.lora_dropout, seed=1234,
                        double_quant=True, grad_checkpointing=True, quantized=args.impl != "bf16", norm_out_fp32=args.norm_out_fp32)
     model.train()
@@ -429,6 +464,9 @@ def run_gpu_arm(args):
         launches = QF.LAUNCH_COUNTER[0]
     t_e2e = timed(loop_e2e, args.steps)
     clocks = sampler.stop() if rank == 0 else {}
+    if args.dump_outputs and rank == 0:   # before the roofline and baseline steps below change the adapters again
+        # --optim torch clips the gradient buffer in place; the paged optimizer applies the clip coefficient in its kernel
+        dump_outputs(args.dump_outputs, static_loss, params, gsync.flat * clip_coef if args.optim == "paged" else gsync.flat)
 
     # roofline of the dominant kernel: CUDA events around every fused launch (same stream), a few more micro-steps
     # (launched eagerly: events cannot be recorded inside a replayed graph)

@@ -24,6 +24,7 @@ from __future__ import annotations
 import math
 import os
 import sys
+import warnings
 from dataclasses import dataclass
 
 import torch
@@ -39,6 +40,13 @@ if _SHIMS not in sys.path:  # `import bitsandbytes` -> shims/bitsandbytes -> qlo
 import bitsandbytes as bnb  # noqa: E402  (the shim; the product package under the reference's import name)
 
 from . import fused_ops  # noqa: E402
+
+try:   # the cuDNN frontend (pip: nvidia-cudnn-frontend) builds the deterministic attention backward (CausalAttention)
+    import cudnn as _cudnn
+except ImportError:
+    _cudnn = None
+    warnings.warn("harness: nvidia-cudnn-frontend is not installed; attention uses torch's SDPA backward, whose dQ is not "
+                  "bit-repeatable, so training steps will differ in the last bits from run to run")
 
 # caller-side elementwise fusions (RoPE on q+k in one launch, SwiGLU fwd/bwd in one launch each); plain torch otherwise
 USE_FUSED_OPS = True
@@ -158,6 +166,62 @@ def _apply_rope(x, cos, sin_signed):
     return torch.addcmul(x * cos, swapped, sin_signed)
 
 
+_CUDNN_HANDLES = {}
+_CUDNN_BWD_GRAPHS = {}
+
+
+def _cudnn_sdpa_backward(q, k, v, o, do, lse):
+    """dQ, dK, dV of causal attention from cuDNN's flash backward with its deterministic algorithm.  The backward PyTorch
+    runs for SDPA accumulates dQ over key blocks with atomics, so the same step would not give the same gradients twice."""
+    cudnn = _cudnn
+    dev = q.device.index
+    if dev not in _CUDNN_HANDLES:
+        with torch.cuda.device(dev):
+            _CUDNN_HANDLES[dev] = cudnn.create_handle()
+    handle = _CUDNN_HANDLES[dev]
+    b, h, s, d = q.shape
+    lse = lse.reshape(b, h, s, 1)
+    if do.stride(-1) != 1:
+        do = do.contiguous()
+    grads = [torch.empty_like(t) for t in (q, k, v)]
+    key = (dev, q.dtype) + tuple((tuple(t.shape), t.stride()) for t in (q, k, v, o, do, lse, *grads))
+    if key not in _CUDNN_BWD_GRAPHS:
+        g = cudnn.pygraph(io_data_type=cudnn.data_type.BFLOAT16, intermediate_data_type=cudnn.data_type.FLOAT,
+                          compute_data_type=cudnn.data_type.FLOAT, handle=handle)
+        ins = [g.tensor_like(t) for t in (q, k, v, o, do, lse)]
+        outs = g.sdpa_backward(*ins, attn_scale=1.0 / math.sqrt(d), use_causal_mask=True, use_deterministic_algorithm=True)
+        for gt, t in zip(outs, grads):
+            gt.set_output(True).set_dim(list(t.shape)).set_stride(list(t.stride())).set_data_type(cudnn.data_type.BFLOAT16)
+        g.validate()
+        g.build_operation_graph()
+        g.create_execution_plans([cudnn.heur_mode.A, cudnn.heur_mode.FALLBACK])
+        g.check_support()
+        g.build_plans()
+        _CUDNN_BWD_GRAPHS[key] = (g, ins + list(outs), g.get_workspace_size())
+    g, tensors, ws = _CUDNN_BWD_GRAPHS[key]
+    workspace = torch.empty(max(ws, 1), device=q.device, dtype=torch.uint8)
+    cudnn.set_stream(handle=handle, stream=torch.cuda.current_stream(q.device).cuda_stream)
+    g.execute(dict(zip(tensors, (q, k, v, o, do, lse, *grads))), workspace, handle=handle)
+    return grads
+
+
+class CausalAttention(torch.autograd.Function):
+    """Causal SDPA on bf16 [b, h, s, d]: the cuDNN flash forward F.scaled_dot_product_attention runs on this GPU, and a
+    backward that gives the same bits on every run (_cudnn_sdpa_backward)."""
+
+    @staticmethod
+    def forward(ctx, q, k, v):
+        assert q.dtype == torch.bfloat16 and q.is_cuda, (q.dtype, q.device)
+        out, lse = torch.ops.aten._scaled_dot_product_cudnn_attention(q, k, v, None, True, 0.0, True, False)[:2]
+        ctx.save_for_backward(q, k, v, out, lse)
+        return out
+
+    @staticmethod
+    def backward(ctx, do):
+        q, k, v, out, lse = (t.detach() for t in ctx.saved_tensors)
+        return tuple(_cudnn_sdpa_backward(q, k, v, out, do.detach(), lse))
+
+
 class DecoderLayer(nn.Module):
     """Submodule names follow HF's LlamaDecoderLayer leaves (q_proj ... down_proj), which is what
     `find_all_linear_names` (qlora.py:248-259) keys on."""
@@ -188,7 +252,7 @@ class DecoderLayer(nn.Module):
             q, k = _apply_rope(q, cos, sin), _apply_rope(k, cos, sin)
         q, k = q.transpose(1, 2), k.transpose(1, 2)
         v = v.view(b, s, self.heads, self.head_dim).transpose(1, 2)
-        a = F.scaled_dot_product_attention(q, k, v, is_causal=True)
+        a = CausalAttention.apply(q, k, v) if _cudnn is not None else F.scaled_dot_product_attention(q, k, v, is_causal=True)
         attn = self.o_proj(a.transpose(1, 2).reshape(b, s, h))
         pn = self.post_attention_layernorm
         if fused and not pn.out_fp32 and x.dtype == torch.bfloat16 and attn.dtype == torch.bfloat16 and h <= 8192 and h % 8 == 0:

@@ -164,3 +164,29 @@ def test_add_rmsnorm_matches_unfused(H, d):
     assert torch.equal(s, s2) and torch.equal(y, y2)
     for a, b in ((x.grad, x2.grad), (dl.grad, d2.grad)):
         assert ((a.float() - b.float()).norm() / b.float().norm()).item() < 4e-3   # one rounding instead of two
+
+
+def test_causal_attention_matches_sdpa_and_repeats(H):
+    """The bench model's attention at the Llama-2-7B shape (seq 2048 = 16 key blocks of the backward, 32 heads of 128): the
+    forward is F.scaled_dot_product_attention's result bit for bit, the gradients agree with its backward up to the order
+    of the dQ sums, and a second backward gives the same bits."""
+    if H._cudnn is None:
+        pytest.skip("nvidia-cudnn-frontend is not installed")
+    g = torch.Generator(device="cuda").manual_seed(0)
+    b, s, h, d = 1, 2048, 32, 128
+    qkv = [torch.randn(b, s, h, d, device="cuda", dtype=torch.bfloat16, generator=g) for _ in range(3)]
+    go = torch.randn(b, s, h, d, device="cuda", dtype=torch.bfloat16, generator=g).transpose(1, 2)
+
+    def run(fn):
+        q, k, v = (t.clone().requires_grad_(True) for t in qkv)
+        o = fn(q.transpose(1, 2), k.transpose(1, 2), v.transpose(1, 2))   # [b, h, s, d] views, as DecoderLayer passes them
+        o.backward(go)
+        return [o.detach(), q.grad, k.grad, v.grad]
+
+    got = run(H.CausalAttention.apply)
+    ref = run(lambda q, k, v: torch.nn.functional.scaled_dot_product_attention(q, k, v, is_causal=True))
+    assert torch.equal(got[0], ref[0])
+    for a, r in zip(got[1:], ref[1:]):
+        assert ((a.float() - r.float()).norm() / r.float().norm()).item() < 1e-3
+    again = run(H.CausalAttention.apply)
+    assert all(torch.equal(a, b) for a, b in zip(got, again))
